@@ -43,6 +43,8 @@ def parse():
     ap.add_argument('--ref-batch', type=int, default=8, help='query images per CPU reference step (bounded sample)')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-graph', action='store_true', help='launch every kernel eagerly instead of replaying a CUDA graph')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs)')
     return ap.parse_args()
 
 
@@ -188,6 +190,43 @@ def cpu_step_factory(ncls, side, B, threads):
         dw[0].sum().backward()
     state['support_only'] = support_only
     return step, state
+
+
+DUMP_SAMPLE = 65536      # values kept per parameter tensor: 89 tensors -> 1.6 M values, 13 MB for params + grads
+DUMP_SEED = 20240
+
+
+def dump_outputs(out_dir, model, region_loss):
+    """What one training step hands its caller, as float32 / float64 .npy files in out_dir:
+      loss.npy          the float32 loss the step returns
+      loss_terms.npy    float64 [x, y, w, h, conf, cls, total] of RegionLossV2 (the reference's log line)
+      counts.npy        float64 [nGT, nCorrect, nProposals]
+      param.<name>.npy  the parameter after the SGD update, flattened in logical (OIHW) order
+      grad.<name>.npy   its gradient, same order
+    Tensors larger than DUMP_SAMPLE values are sampled at sorted positions drawn from a generator seeded with
+    (DUMP_SEED, parameter index), so two runs or two builds sample the same positions."""
+    os.makedirs(out_dir, exist_ok=True)
+
+    def save(name, a):
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+    losses = region_loss.last['losses'].cpu().numpy()
+    counters = region_loss.last['counters'].cpu().numpy()
+    save('loss', losses[6].astype(np.float32))     # the returned loss is losses[6] cast to float32
+    save('loss_terms', losses[:7])
+    save('counts', np.array([counters[0], counters[1], losses[7]], dtype=np.float64))
+    for i, (name, p) in enumerate(model.named_parameters()):
+        n = p.numel()
+        idx = None
+        if n > DUMP_SAMPLE:
+            pos = np.sort(np.random.default_rng([DUMP_SEED, i]).choice(n, DUMP_SAMPLE, replace=False))
+            idx = torch.from_numpy(pos).to(p.device)
+        for tag, t in (('param', p), ('grad', p.grad)):
+            if t is None:
+                continue
+            v = t.detach().reshape(-1)
+            if idx is not None:
+                v = v[idx]
+            save('%s.%s' % (tag, name), v.float().cpu().numpy())
 
 
 def fair_cpu_rate(B_ref, B_full, t_step, t_support):
@@ -408,6 +447,8 @@ def main():
     ms = timed(lambda i: step(*resident[i % 2]), args.steps, 'value')
     clocks = sampler.stop() if rank == 0 else None
     value = global_batch * args.steps / (ms / 1e3)
+    if args.dump_outputs and rank == 0:     # before the untimed steps below move the parameters on
+        dump_outputs(args.dump_outputs, model, region_loss)
 
     # per-kernel timing + launch count: the same kernels launched eagerly (a CUDA-graph replay has no per-kernel
     # CUDA events), in the same run, right after the timed region

@@ -88,10 +88,13 @@ def test_layers():
     assert np.array_equal(y.numpy(), d['dyn_out'])
 
 
-def _run_meta(d, det, ler, regen_inputs):
+def _run_meta(d, det, ler, regen_inputs, double=False):
+    """double: the network in float64, the region loss in float32 on the cast head output (as in the reference)."""
     seed = int(d['seed'])
     m = ODK.MetaDarknet(det, ler)
     seeded_init(m, seed)
+    if double:
+        m.double()
     m.train()
     bs, cs, side, ms = int(d['bs']), int(d['cs']), int(d['side']), int(d['meta_side'])
     if regen_inputs:
@@ -101,10 +104,15 @@ def _run_meta(d, det, ler, regen_inputs):
         mask = torch.from_numpy(synth_masks(cs, ms, seed + 2))
     else:
         x, metax, mask = (torch.from_numpy(d[k]) for k in ('x', 'metax', 'mask'))
+    if double:
+        x, metax, mask = x.double(), metax.double(), mask.double()
     out = m(x, metax, mask)
-    loss = ORL.region_loss_v2(out, torch.from_numpy(d['target']), m.anchors, m.num_anchors, m.num_classes,
+    o = out.detach().float().requires_grad_(True) if double else out
+    loss = ORL.region_loss_v2(o, torch.from_numpy(d['target']), m.anchors, m.num_anchors, m.num_classes,
                               seen=int(d['seen']))
     loss.backward()
+    if double:
+        out.backward(o.grad.double())
     return m, out, loss
 
 
@@ -132,10 +140,17 @@ def test_meta_full416_digest():
     m, out, loss = _run_meta(d, netcfg.darknet_dynamic_blocks(), netcfg.reweighting_net_blocks(), True)
     assert rel(out.detach().numpy(), d['output']) < 1e-5
     assert abs(loss.item() - float(d['loss'])) < 1e-5 * abs(float(d['loss']))
+    # The float32 gradients of the full-size network move by up to ~4e-3 with the CPU's convolution kernels (thread
+    # count, instruction set), so they are compared with the reference's float64 run (tests/golden/meta_full416_f64.npz)
+    # instead: the oracle stays 7e-10 (norm) and 5e-9 (first values) from it with AVX2 or AVX-512 kernels, any thread count.
+    d = load('meta_full416_f64.npz')
+    m, out, loss = _run_meta(d, netcfg.darknet_dynamic_blocks(), netcfg.reweighting_net_blocks(), True, double=True)
+    assert rel(out.detach().numpy(), d['output']) < 1e-10
+    assert abs(loss.item() - float(d['loss'])) < 1e-6 * abs(float(d['loss']))
     for name, p in m.named_parameters():
         gn = float(d['gradnorm/' + name])
-        assert abs(p.grad.double().norm().item() - gn) < 1e-4 * gn + 1e-12, name
-        assert rel(p.grad.reshape(-1)[:64].numpy(), d['gradhead/' + name]) < 1e-3, name
+        assert abs(p.grad.norm().item() - gn) < 1e-7 * gn + 1e-12, name
+        assert rel(p.grad.reshape(-1)[:64].numpy(), d['gradhead/' + name]) < 1e-6, name
 
 
 def test_tiny_yolo_416_config1():
