@@ -31,6 +31,8 @@ SIGNATURES = {
     'fsdet_conv_first_fwd_stats': ('pipippiiiiipp', 'i'),
     'fsdet_conv_first_wgrad': ('pipipippziiiip', 'i'),
     'fsdet_conv_first_wgrad_workspace_floats': ('iiii', 'z'),
+    'fsdet_conv_first_wgrad_workspace_floats_cin': ('iiiii', 'z'),
+    'fsdet_conv_first_wgrad_supported': ('ii', 'i'),
     'fsdet_conv_first_tc_supported': ('iii', 'i'),
     'fsdet_conv_first_tc_rows': ('iii', 'i'),
     'fsdet_conv_first_tc_stats': ('pipipppiiiip', 'i'),
@@ -83,6 +85,7 @@ SIGNATURES = {
     'fsdet_rw_running_mean': ('pppppiiip', 'i'),
     'fsdet_augment_workspace_bytes': ('iiii', 'z'),
     'fsdet_augment_batch': ('pppiiiiipzpppp', 'i'),
+    'fsdet_augment_batch_pitched': ('pppiiiiipzpzppp', 'i'),
     'fsdet_box_masks': ('piiipp', 'i'),
 }
 

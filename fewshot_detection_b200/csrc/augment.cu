@@ -186,9 +186,10 @@ struct AugArgs {
     const int32_t* geom;        // [n][8]
     const int32_t* tables;      // [n][2][L][2 + kmax]
     const uint8_t* luts;        // [n][3][256]
-    float* out;                 // [n][3][H][W]
+    float* out;                 // [n][3][H][W], image i at out + i * out_pitch
     uint8_t* out_u8;            // optional [n][H][W][3]: the uint8 image before ToTensor (what PIL would hold)
     int n, W, H, L, kmax, filter;
+    long long out_pitch;        // floats from one image's output to the next (>= 3*H*W)
 };
 
 // cropped pixel (x, y) of image.py:72: zero outside the source
@@ -278,7 +279,7 @@ __global__ void __launch_bounds__(kAugThreads) augment_kernel(AugArgs p) {
     }
     const int ox = flip ? p.W - 1 - xx : xx;  // Image.FLIP_LEFT_RIGHT (colour ops are per pixel: order is irrelevant)
     const size_t plane = (size_t)p.W * p.H;
-    float* o = p.out + (size_t)img * 3 * plane + (size_t)yy * p.W + ox;
+    float* o = p.out + (size_t)img * p.out_pitch + (size_t)yy * p.W + ox;
     o[0] = __fdiv_rn((float)r, 255.f);
     o[plane] = __fdiv_rn((float)gg, 255.f);
     o[2 * plane] = __fdiv_rn((float)b, 255.f);
@@ -317,8 +318,17 @@ extern "C" size_t fsdet_augment_workspace_bytes(int n, int W, int H, int kmax) {
 extern "C" int fsdet_augment_batch(const uint8_t* const* src, const int32_t* geom, const double* color, int n, int W,
                                    int H, int kmax, int filter, void* workspace, size_t workspace_bytes, float* out,
                                    uint8_t* out_u8, int32_t* status, void* stream) {
+    FSDET_CHECK_ARG(W > 0 && H > 0, "augment_batch: bad shape");
+    return fsdet_augment_batch_pitched(src, geom, color, n, W, H, kmax, filter, workspace, workspace_bytes, out,
+                                       (size_t)3 * W * H, out_u8, status, stream);
+}
+
+extern "C" int fsdet_augment_batch_pitched(const uint8_t* const* src, const int32_t* geom, const double* color, int n, int W,
+                                           int H, int kmax, int filter, void* workspace, size_t workspace_bytes, float* out,
+                                           size_t out_pitch, uint8_t* out_u8, int32_t* status, void* stream) {
     FSDET_CHECK_ARG(src && geom && color && workspace && out && status, "augment_batch: null pointer");
     FSDET_CHECK_ARG(n >= 0 && W > 0 && H > 0, "augment_batch: bad shape");
+    FSDET_CHECK_ARG(out_pitch >= (size_t)3 * W * H, "augment_batch: output pitch %zu < 3*H*W", out_pitch);
     FSDET_CHECK_ARG(filter == 0 || filter == 3, "augment_batch: filter %d (0 = NEAREST, 3 = BICUBIC)", filter);
     FSDET_CHECK_ARG(kmax >= 1 && kmax <= 254, "augment_batch: kmax %d (1..254)", kmax);
     FSDET_CHECK_ARG(workspace_bytes >= fsdet_augment_workspace_bytes(n, W, H, kmax) && aligned16(workspace),
@@ -337,7 +347,7 @@ extern "C" int fsdet_augment_batch(const uint8_t* const* src, const int32_t* geo
     if (st) return st;
     AugArgs p;
     p.src = src; p.geom = geom; p.tables = tables; p.luts = luts; p.out = out; p.out_u8 = out_u8;
-    p.n = n; p.W = W; p.H = H; p.L = L; p.kmax = kmax; p.filter = filter;
+    p.n = n; p.W = W; p.H = H; p.L = L; p.kmax = kmax; p.filter = filter; p.out_pitch = (long long)out_pitch;
     augment_kernel<<<dim3(ceil_div((long long)W * H, kAugThreads), n), kAugThreads, 0, s>>>(p);
     return launch_status("augment");
 }

@@ -474,11 +474,12 @@ __device__ __forceinline__ void cp_async16_zfill(void* smem_dst, const float* sr
 }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
-// forward: lane = output channel (its 9x4 filter lives in registers as pairs), one warp walks along an image row
-// keeping the 3x3 input window in registers (3 broadcast shared-memory loads + 36 FMAs per pixel, one coalesced
+// forward: lane = output channel (its 9x(4*NQ) filter lives in registers as pairs), one warp walks along an image row
+// keeping the 3x3 input window in registers (3*NQ broadcast shared-memory loads + 36*NQ FMAs per pixel, one coalesced
 // 128-byte store).  The walk is unrolled by three so the window rotates by renaming, not by moves.  Persistent CTAs
 // (two per SM) loop over tiles of FT_H rows (one per warp) x FT_W columns; the next tile's input is fetched with
 // asynchronous copies into the other half of a double buffer while the current one is being computed.
+// NQ = channel quads per pixel: 1 for <= 4 input channels (image + mask), 2 for 5..8 (image + cropped object [+ mask]).
 constexpr int FT_H = 8, FT_W = 104, FT_NPX = (FT_H + 2) * (FT_W + 2);
 template <bool PK> struct Px4 { Pair<PK> lo, hi; };   // one pixel: channels (0,1) and (2,3)
 template <bool PK> __device__ __forceinline__ Px4<PK> lds_px(const float4* p) {
@@ -486,16 +487,30 @@ template <bool PK> __device__ __forceinline__ Px4<PK> lds_px(const float4* p) {
     Px4<PK> r; r.lo = Pair<PK>::raw(v.x); r.hi = Pair<PK>::raw(v.y);
     return r;
 }
+template <bool PK, int NQ> struct PxN { Px4<PK> q[NQ]; };   // one pixel: NQ channel quads
+template <bool PK, int NQ> __device__ __forceinline__ PxN<PK, NQ> lds_pxn(const float4* p) {
+    PxN<PK, NQ> r;
+#pragma unroll
+    for (int q = 0; q < NQ; ++q) r.q[q] = lds_px<PK>(p + q);
+    return r;
+}
+// input tile bytes of the 8-channel forward (double buffered): above the 48 KB static limit, so dynamic shared memory
+constexpr int first_fwd_smem_bytes(int nq) { return 2 * FT_NPX * nq * (int)sizeof(float4); }
 // STATS: the BatchNorm partial row of this CTA (sum | sum of squares | min | max per channel, the layout
 // fsdet_bn_finalize reads) is taken from the values while they are in registers - a thread owns ONE output channel, so
 // there is nothing to transpose - instead of a separate pass over the 1.4 GB tensor (fsdet_colstats).
-// (two CTAs per SM at 122 registers; three at 80 registers measured slower: 1.12 vs 1.02 ms per step, tools/r2b_callE.sh)
-template <bool PK, bool STATS>
-__global__ void __launch_bounds__(256, 2) conv_first_fwd_kernel(const float* __restrict__ in0, int C0, const float* __restrict__ in1,
-                                                                int C1, const float* __restrict__ w /* [Cout][9][4] */,
+// (NQ = 1: two CTAs per SM at 122 registers; three at 80 registers measured slower: 1.12 vs 1.02 ms per step,
+// tools/r2b_callE.sh.  NQ = 2 holds twice the weights and window: one CTA per SM, no spills.)
+template <bool PK, bool STATS, int NQ>
+__global__ void __launch_bounds__(256, NQ == 1 ? 2 : 1) conv_first_fwd_kernel(const float* __restrict__ in0, int C0,
+                                                                const float* __restrict__ in1,
+                                                                int C1, const float* __restrict__ w /* [Cout][9][4*NQ] */,
                                                                 float* __restrict__ z, int ldz, int B, int H, int W, int Cout,
                                                                 float* __restrict__ stats) {
-    __shared__ float4 xs[2][FT_NPX];
+    typedef float4 Tile[FT_NPX * NQ];                   // one buffer: [FT_NPX pixels][NQ quads]
+    __shared__ float4 xs_static[NQ == 1 ? 2 : 1][NQ == 1 ? FT_NPX : 1];
+    extern __shared__ __align__(16) float4 xs_dyn[];
+    Tile* const xs = NQ == 1 ? reinterpret_cast<Tile*>(xs_static) : reinterpret_cast<Tile*>(xs_dyn);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int tiles_w = (W + FT_W - 1) / FT_W, tiles_h = (H + FT_H - 1) / FT_H;
     const int tiles = B * tiles_h * tiles_w;
@@ -516,10 +531,10 @@ __global__ void __launch_bounds__(256, 2) conv_first_fwd_kernel(const float* __r
         for (int r = warp; r < FT_H + 2; r += 8) {
             const int h = h0 + r - 1;
             const bool rok = h >= 0 && h < H;
-            const unsigned dst = (unsigned)__cvta_generic_to_shared(&xs[buf][r * (FT_W + 2) + lane]);
+            const unsigned dst = (unsigned)__cvta_generic_to_shared(&xs[buf][(r * (FT_W + 2) + lane) * NQ]);
             const long long off = (long long)(rok ? h : 0) * W + (w0 - 1 + lane);
 #pragma unroll
-            for (int ch = 0; ch < 4; ++ch) {
+            for (int ch = 0; ch < 4 * NQ; ++ch) {
                 const float* plane = ch < C0 ? in0 + ((long long)b * C0 + ch) * HW
                                              : (ch < C0 + C1 ? in1 + ((long long)b * C1 + (ch - C0)) * HW : nullptr);
                 const bool pok = rok && plane != nullptr;
@@ -528,18 +543,23 @@ __global__ void __launch_bounds__(256, 2) conv_first_fwd_kernel(const float* __r
                 for (int j = 0; j < 4; ++j) {
                     if (lane + 32 * j < FT_W + 2) {
                         const bool ok = pok && cok_[j];
-                        asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;" ::"r"(dst + (32 * j * 4 + ch) * 4),
+                        asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;" ::"r"(dst + (32 * j * 4 * NQ + ch) * 4),
                                      "l"(ok ? src + 32 * j : in0), "r"(ok ? 4 : 0) : "memory");
                     }
                 }
             }
         }
     };
-    Px4<PK> wr[9];
+    static_assert(NQ == 1 || NQ == 2, "up to 8 input channels");
+    PxN<PK, NQ> wr[9];
 #pragma unroll
     for (int k = 0; k < 9; ++k) {
-        const float4 v = lane < Cout ? ldg4(w + (lane * 9 + k) * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
-        wr[k].lo = Pair<PK>::make(v.x, v.y); wr[k].hi = Pair<PK>::make(v.z, v.w);
+        const float4 v = lane < Cout ? ldg4(w + (lane * 9 + k) * 4 * NQ) : make_float4(0.f, 0.f, 0.f, 0.f);
+        wr[k].q[0].lo = Pair<PK>::make(v.x, v.y); wr[k].q[0].hi = Pair<PK>::make(v.z, v.w);
+        if (NQ == 2) {
+            const float4 u = lane < Cout ? ldg4(w + (lane * 9 + k) * 4 * NQ + 4) : make_float4(0.f, 0.f, 0.f, 0.f);
+            wr[k].q[NQ - 1].lo = Pair<PK>::make(u.x, u.y); wr[k].q[NQ - 1].hi = Pair<PK>::make(u.z, u.w);
+        }
     }
     const bool cok = lane < Cout;
     float tsum = 0.f, esum = 0.f, tsq = 0.f, esq = 0.f, tmn = INFINITY, tmx = -INFINITY;   // this thread's channel, all its pixels
@@ -556,19 +576,22 @@ __global__ void __launch_bounds__(256, 2) conv_first_fwd_kernel(const float* __r
         const int h = th * FT_H + warp, w0 = tw * FT_W;
         if (h >= H) continue;
         const int wn = min(FT_W, W - w0);
-        const float4* r0 = &xs[buf][warp * (FT_W + 2)];
-        const float4* r1 = r0 + (FT_W + 2);
-        const float4* r2 = r1 + (FT_W + 2);
+        const float4* r0 = &xs[buf][warp * (FT_W + 2) * NQ];
+        const float4* r1 = r0 + (FT_W + 2) * NQ;
+        const float4* r2 = r1 + (FT_W + 2) * NQ;
         float* zr = z + (((long long)b * H + h) * W + w0) * ldz + lane;
         // window columns: P = c, Q = c + 1, R = c + 2 (rows 0..2)
-        Px4<PK> p0 = lds_px<PK>(r0), p1 = lds_px<PK>(r1), p2 = lds_px<PK>(r2);
-        Px4<PK> q0 = lds_px<PK>(r0 + 1), q1 = lds_px<PK>(r1 + 1), q2 = lds_px<PK>(r2 + 1);
-        Px4<PK> s0, s1, s2;
-#define FSDET_TAP(X, K) alo.fma(X.lo, wr[K].lo); ahi.fma(X.hi, wr[K].hi);
+        PxN<PK, NQ> p0 = lds_pxn<PK, NQ>(r0), p1 = lds_pxn<PK, NQ>(r1), p2 = lds_pxn<PK, NQ>(r2);
+        PxN<PK, NQ> q0 = lds_pxn<PK, NQ>(r0 + NQ), q1 = lds_pxn<PK, NQ>(r1 + NQ), q2 = lds_pxn<PK, NQ>(r2 + NQ);
+        PxN<PK, NQ> s0, s1, s2;
+#define FSDET_TAP(X, K)                                                                                   \
+    alo.fma(X.q[0].lo, wr[K].q[0].lo); ahi.fma(X.q[0].hi, wr[K].q[0].hi);                                 \
+    if (NQ == 2) { alo.fma(X.q[NQ - 1].lo, wr[K].q[NQ - 1].lo); ahi.fma(X.q[NQ - 1].hi, wr[K].q[NQ - 1].hi); }
 #define FSDET_PIXEL(A0, A1, A2, B0, B1, B2, C0_, C1_, C2_, COL)                                           \
     {                                                                                                     \
-        C0_ = lds_px<PK>(r0 + (COL) + 2); C1_ = lds_px<PK>(r1 + (COL) + 2); C2_ = lds_px<PK>(r2 + (COL) + 2); \
-        Pair<PK> alo = Pair<PK>::make(0.f, 0.f), ahi = alo;   /* one accumulator per input channel */      \
+        C0_ = lds_pxn<PK, NQ>(r0 + (COL) * NQ + 2 * NQ); C1_ = lds_pxn<PK, NQ>(r1 + (COL) * NQ + 2 * NQ);  \
+        C2_ = lds_pxn<PK, NQ>(r2 + (COL) * NQ + 2 * NQ);                                                  \
+        Pair<PK> alo = Pair<PK>::make(0.f, 0.f), ahi = alo;   /* one accumulator per channel of a quad */  \
         FSDET_TAP(A0, 0) FSDET_TAP(B0, 1) FSDET_TAP(C0_, 2)                                                \
         FSDET_TAP(A1, 3) FSDET_TAP(B1, 4) FSDET_TAP(C1_, 5)                                                \
         FSDET_TAP(A2, 6) FSDET_TAP(B2, 7) FSDET_TAP(C2_, 8)                                                \
@@ -622,28 +645,41 @@ __global__ void __launch_bounds__(256, 2) conv_first_fwd_kernel(const float* __r
 // x row per step, three at an image boundary); the next row is fetched with asynchronous copies while the current
 // one is computed.  Thread (co, filter row ty, column segment) keeps the 3 taps of its filter row x 4 input channels
 // in registers and slides a 3-pixel window along its segment of the image row (one new x pixel + one dz value per
-// step feed 12 FMAs); partials are reduced in a fixed order afterwards.
-constexpr int FW_SEG = 6;                       // column segments per row (thread groups)
-constexpr int FW_THREADS = 32 * 3 * FW_SEG;
+// step feed 12 FMAs per channel quad); partials are reduced in a fixed order afterwards.  NQ = channel quads, as in the
+// forward.
+// column segments per row (thread groups): 6 for one channel quad; 5 for two, whose 15 warps leave each thread the
+// 128 registers that its 24 accumulators and 3-pixel window need without spilling (18 warps allow 96)
+template <int NQ> struct FirstWgrad {
+    static constexpr int SEG = NQ == 1 ? 6 : 5;
+    static constexpr int THREADS = 32 * 3 * SEG;
+};
+constexpr int first_wgrad_seg(int nq) { return nq == 1 ? FirstWgrad<1>::SEG : FirstWgrad<2>::SEG; }
 constexpr int FW_SLOTS = 6;
-template <bool PK>
-__global__ void __launch_bounds__(FW_THREADS, 1) conv_first_wgrad_kernel(const float* __restrict__ in0, int C0,
+// shared-memory bytes of the weight-gradient kernel: the x ring and the double-buffered dz row
+constexpr size_t first_wgrad_smem_bytes(int nq, int W) {
+    return ((size_t)FW_SLOTS * (W + 2) * 4 * nq + (size_t)2 * W * 32) * sizeof(float);
+}
+template <bool PK, int NQ>
+__global__ void __launch_bounds__(FirstWgrad<NQ>::THREADS, 1) conv_first_wgrad_kernel(const float* __restrict__ in0, int C0,
                                                                          const float* __restrict__ in1, int C1,
                                                                          const float* __restrict__ dz, int lddz,
                                                                          float* __restrict__ part, int B, int H, int W, int Cout) {
     extern __shared__ __align__(16) float sm[];
-    float4* xs = reinterpret_cast<float4*>(sm);              // [FW_SLOTS][W + 2] pixels of 4 channels (zero halo)
-    float* ds = sm + FW_SLOTS * (W + 2) * 4;                 // [2][W][32]
+    float4* xs = reinterpret_cast<float4*>(sm);              // [FW_SLOTS][W + 2] pixels of 4*NQ channels (zero halo)
+    float* ds = sm + FW_SLOTS * (W + 2) * 4 * NQ;            // [2][W][32]
     const int tid = threadIdx.x;
     const int co = tid & 31;
     const int ty = (tid >> 5) % 3;                           // filter row
+    constexpr int FW_SEG = FirstWgrad<NQ>::SEG, FW_THREADS = FirstWgrad<NQ>::THREADS;
     const int seg = (tid >> 5) / 3;                          // column segment 0..FW_SEG-1
     const int wseg = (W + FW_SEG - 1) / FW_SEG;
     const int wbeg = seg * wseg, wend = min(W, wbeg + wseg);
     const int HW = H * W;
-    Pair<PK> acc[3][2];                                      // taps (ty, 0..2) x channel pairs
+    Pair<PK> acc[3][2 * NQ];                                 // taps (ty, 0..2) x channel pairs
 #pragma unroll
-    for (int i = 0; i < 3; ++i) acc[i][0] = acc[i][1] = Pair<PK>::make(0.f, 0.f);
+    for (int i = 0; i < 3; ++i)
+#pragma unroll
+        for (int q = 0; q < 2 * NQ; ++q) acc[i][q] = Pair<PK>::make(0.f, 0.f);
     const long long rows = (long long)B * H;
     const long long per = (rows + gridDim.x - 1) / gridDim.x;
     const long long rbeg = (long long)blockIdx.x * per, rend = min(rows, rbeg + per);
@@ -658,11 +694,11 @@ __global__ void __launch_bounds__(FW_THREADS, 1) conv_first_wgrad_kernel(const f
             const bool cok_ = c >= 1 && c <= W;
             for (int k = 3 - nnew; k < 3; ++k) {
                 const int q = h - 1 + k;
-                const unsigned dst = (unsigned)__cvta_generic_to_shared(xs + ((win + k) % FW_SLOTS) * (W + 2) + c);
+                const unsigned dst = (unsigned)__cvta_generic_to_shared(xs + ((win + k) % FW_SLOTS) * (W + 2) * NQ + c * NQ);
                 const bool ok = cok_ && q >= 0 && q < H;
                 const long long off = (long long)(ok ? q : 0) * W + (c - 1);
 #pragma unroll
-                for (int ch = 0; ch < 4; ++ch) {
+                for (int ch = 0; ch < 4 * NQ; ++ch) {
                     const float* plane = ch < C0 ? in0 + ((long long)b * C0 + ch) * HW
                                                  : (ch < C0 + C1 ? in1 + ((long long)b * C1 + (ch - C0)) * HW : nullptr);
                     const bool okc = ok && plane != nullptr;
@@ -690,18 +726,19 @@ __global__ void __launch_bounds__(FW_THREADS, 1) conv_first_wgrad_kernel(const f
         __syncthreads();            // this row has landed; everyone is done with the previous one
         const int wcur = win;
         if (row + 1 < rend) stage(row + 1, buf ^ 1);
-        const float4* xr = xs + ((wcur + ty) % FW_SLOTS) * (W + 2);   // image row h + ty - 1;  xr[w + tx] = x[.][w + tx - 1]
+        const float4* xr = xs + ((wcur + ty) % FW_SLOTS) * (W + 2) * NQ;   // image row h + ty - 1;  xr[(w + tx) NQ] = x[.][w + tx - 1]
         const float* dcur = ds + buf * W * 32 + co;
         if (wbeg < wend) {
-            Px4<PK> x0 = lds_px<PK>(xr + wbeg), x1 = lds_px<PK>(xr + wbeg + 1), x2;
+            PxN<PK, NQ> x0 = lds_pxn<PK, NQ>(xr + wbeg * NQ), x1 = lds_pxn<PK, NQ>(xr + wbeg * NQ + NQ), x2;
+#define FSDET_MAC(I, X)                                                                          \
+    acc[I][0].fma(dd, X.q[0].lo); acc[I][1].fma(dd, X.q[0].hi);                                  \
+    if (NQ == 2) { acc[I][2 * NQ - 2].fma(dd, X.q[NQ - 1].lo); acc[I][2 * NQ - 1].fma(dd, X.q[NQ - 1].hi); }
 #define FSDET_STEP(X0, X1, X2, WW)                                                               \
     {                                                                                            \
-        X2 = lds_px<PK>(xr + (WW) + 2);                                                          \
+        X2 = lds_pxn<PK, NQ>(xr + (WW) * NQ + 2 * NQ);                                           \
         const float d = dcur[(WW) * 32];                                                         \
         const Pair<PK> dd = Pair<PK>::make(d, d);                                                \
-        acc[0][0].fma(dd, X0.lo); acc[0][1].fma(dd, X0.hi);                                      \
-        acc[1][0].fma(dd, X1.lo); acc[1][1].fma(dd, X1.hi);                                      \
-        acc[2][0].fma(dd, X2.lo); acc[2][1].fma(dd, X2.hi);                                      \
+        FSDET_MAC(0, X0) FSDET_MAC(1, X1) FSDET_MAC(2, X2)                                       \
     }
             int w = wbeg;
 #pragma unroll 1
@@ -715,15 +752,18 @@ __global__ void __launch_bounds__(FW_THREADS, 1) conv_first_wgrad_kernel(const f
                 if (w + 1 < wend) FSDET_STEP(x1, x2, x0, w + 1)
             }
 #undef FSDET_STEP
+#undef FSDET_MAC
         }
     }
     if (co < Cout) {
-        float* dst = part + (((long long)blockIdx.x * FW_SEG + seg) * Cout + co) * 36 + ty * 12;
+        float* dst = part + (((long long)blockIdx.x * FW_SEG + seg) * Cout + co) * 36 * NQ + ty * 12 * NQ;
 #pragma unroll
-        for (int i = 0; i < 3; ++i) {
-            const float2 l = acc[i][0].get(), u = acc[i][1].get();
-            *reinterpret_cast<float4*>(dst + 4 * i) = make_float4(l.x, l.y, u.x, u.y);
-        }
+        for (int i = 0; i < 3; ++i)
+#pragma unroll
+            for (int q = 0; q < NQ; ++q) {
+                const float2 l = acc[i][2 * q].get(), u = acc[i][2 * q + 1].get();
+                *reinterpret_cast<float4*>(dst + 4 * (i * NQ + q)) = make_float4(l.x, l.y, u.x, u.y);
+            }
     }
 }
 
@@ -859,22 +899,49 @@ static int first_wgrad_ctas(int B, int H) {
     return (int)(rows < n ? rows : n);
 }
 
+static int first_quads(int C) { return C <= 4 ? 1 : 2; }   // weight / dw channel pitch 4 * quads
+
 extern "C" size_t fsdet_conv_first_wgrad_workspace_floats(int B, int H, int W, int Cout) {
-    (void)W;
-    return (size_t)first_wgrad_ctas(B, H) * FW_SEG * Cout * 36;
+    return fsdet_conv_first_wgrad_workspace_floats_cin(B, H, W, 4, Cout);
 }
 
-extern "C" int fsdet_conv_first_fwd(const float* in0, int C0, const float* in1, int C1, const float* w_pad4, float* z, int ldz,
+extern "C" size_t fsdet_conv_first_wgrad_workspace_floats_cin(int B, int H, int W, int Cin, int Cout) {
+    (void)W;
+    const int nq = first_quads(Cin);
+    return (size_t)first_wgrad_ctas(B, H) * first_wgrad_seg(nq) * Cout * 36 * nq;
+}
+
+extern "C" int fsdet_conv_first_wgrad_supported(int Cin, int W) {
+    return Cin >= 1 && Cin <= 8 && W > 0 && first_wgrad_smem_bytes(first_quads(Cin), W) <= 227 * 1024;
+}
+
+template <bool STATS, int NQ>
+static int launch_first_fwd(const float* in0, int C0, const float* in1, int C1, const float* w, float* z, int ldz, int B, int H,
+                            int W, int Cout, float* stats, unsigned ctas, cudaStream_t s) {
+    // packed FFMA2 flavour: fewer issue slots per pixel (measured 705 us vs 750 us at B=64, 416x416, 4 channels)
+    auto kern = conv_first_fwd_kernel<true, STATS, NQ>;
+    const int smem = NQ == 1 ? 0 : first_fwd_smem_bytes(NQ);
+    if (NQ > 1) {   // dynamic shared-memory opt-in per launch, as conv_first_wgrad
+        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        if (e != cudaSuccess) { set_error("conv_first_fwd: %s", cudaGetErrorString(e)); return (int)e; }
+    }
+    kern<<<ctas, 256, smem, s>>>(in0, C0, in1, C1, w, z, ldz, B, H, W, Cout, stats);
+    return 0;
+}
+
+extern "C" int fsdet_conv_first_fwd(const float* in0, int C0, const float* in1, int C1, const float* w_pad, float* z, int ldz,
                                     int B, int H, int W, int Cout, void* stream) {
-    FSDET_CHECK_ARG(in0 && w_pad4 && z && C0 > 0 && C1 >= 0 && (C1 == 0 || in1) && C0 + C1 <= 4, "conv_first_fwd: bad inputs");
-    FSDET_CHECK_ARG(Cout > 0 && Cout <= 32 && Cout % 4 == 0 && ldz % 4 == 0 && aligned16(z) && aligned16(w_pad4),
+    FSDET_CHECK_ARG(in0 && w_pad && z && C0 > 0 && C1 >= 0 && (C1 == 0 || in1) && C0 + C1 <= 8, "conv_first_fwd: bad inputs");
+    FSDET_CHECK_ARG(Cout > 0 && Cout <= 32 && Cout % 4 == 0 && ldz % 4 == 0 && aligned16(z) && aligned16(w_pad),
                     "conv_first_fwd: Cout=%d ldz=%d", Cout, ldz);
     long long tiles = (long long)B * ceil_div(H, FT_H) * ceil_div(W, FT_W);
     if (tiles == 0) return 0;
     FSDET_CHECK_ARG(tiles < (1ll << 31), "conv_first_fwd: too many tiles");
     const unsigned ctas = (unsigned)(tiles < 2LL * kNumSMs ? tiles : 2LL * kNumSMs);
-    // packed FFMA2 flavour: fewer issue slots per pixel (measured 705 us vs 750 us at B=64, 416x416)
-    conv_first_fwd_kernel<true, false><<<ctas, 256, 0, (cudaStream_t)stream>>>(in0, C0, in1, C1, w_pad4, z, ldz, B, H, W, Cout, nullptr);
+    const int e = first_quads(C0 + C1) == 1
+        ? launch_first_fwd<false, 1>(in0, C0, in1, C1, w_pad, z, ldz, B, H, W, Cout, nullptr, ctas, (cudaStream_t)stream)
+        : launch_first_fwd<false, 2>(in0, C0, in1, C1, w_pad, z, ldz, B, H, W, Cout, nullptr, ctas, (cudaStream_t)stream);
+    if (e) return e;
     return launch_status("conv_first_fwd");
 }
 
@@ -883,44 +950,58 @@ extern "C" int fsdet_conv_first_stat_rows(int B, int H, int W) {
     return (int)(tiles < 2LL * kNumSMs ? tiles : 2LL * kNumSMs);
 }
 
-extern "C" int fsdet_conv_first_fwd_stats(const float* in0, int C0, const float* in1, int C1, const float* w_pad4, float* z, int ldz,
+extern "C" int fsdet_conv_first_fwd_stats(const float* in0, int C0, const float* in1, int C1, const float* w_pad, float* z, int ldz,
                                           int B, int H, int W, int Cout, float* stat_partial, void* stream) {
-    FSDET_CHECK_ARG(in0 && w_pad4 && z && stat_partial && C0 > 0 && C1 >= 0 && (C1 == 0 || in1) && C0 + C1 <= 4,
+    FSDET_CHECK_ARG(in0 && w_pad && z && stat_partial && C0 > 0 && C1 >= 0 && (C1 == 0 || in1) && C0 + C1 <= 8,
                     "conv_first_fwd_stats: bad inputs");
-    FSDET_CHECK_ARG(Cout > 0 && Cout <= 32 && Cout % 4 == 0 && ldz % 4 == 0 && aligned16(z) && aligned16(w_pad4),
+    FSDET_CHECK_ARG(Cout > 0 && Cout <= 32 && Cout % 4 == 0 && ldz % 4 == 0 && aligned16(z) && aligned16(w_pad),
                     "conv_first_fwd_stats: Cout=%d ldz=%d", Cout, ldz);
     long long tiles = (long long)B * ceil_div(H, FT_H) * ceil_div(W, FT_W);
     if (tiles == 0) return 0;
     FSDET_CHECK_ARG(tiles < (1ll << 31), "conv_first_fwd_stats: too many tiles");
     const unsigned ctas = (unsigned)fsdet_conv_first_stat_rows(B, H, W);
-    conv_first_fwd_kernel<true, true><<<ctas, 256, 0, (cudaStream_t)stream>>>(in0, C0, in1, C1, w_pad4, z, ldz, B, H, W, Cout,
-                                                                              stat_partial);
+    const int e = first_quads(C0 + C1) == 1
+        ? launch_first_fwd<true, 1>(in0, C0, in1, C1, w_pad, z, ldz, B, H, W, Cout, stat_partial, ctas, (cudaStream_t)stream)
+        : launch_first_fwd<true, 2>(in0, C0, in1, C1, w_pad, z, ldz, B, H, W, Cout, stat_partial, ctas, (cudaStream_t)stream);
+    if (e) return e;
     return launch_status("conv_first_fwd_stats");
+}
+
+template <int NQ>
+static int launch_first_wgrad(const float* in0, int C0, const float* in1, int C1, const float* dz, int lddz, float* ws, int B,
+                              int H, int W, int Cout, int ctas, cudaStream_t s) {
+    auto kern = conv_first_wgrad_kernel<false, NQ>;
+    {   // the opt-in ceiling (227 KB), per launch like every other kernel of the library: no cached state, and never lowered under
+        // a graph that was captured at a wider image
+        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+        if (e != cudaSuccess) { set_error("conv_first_wgrad: %s", cudaGetErrorString(e)); return (int)e; }
+    }
+    // scalar FFMA flavour (the packed one is register-bandwidth bound here: 900 us vs 873 us)
+    kern<<<ctas, FirstWgrad<NQ>::THREADS, first_wgrad_smem_bytes(NQ, W), s>>>(in0, C0, in1, C1, dz, lddz, ws, B, H, W, Cout);
+    return 0;
 }
 
 extern "C" int fsdet_conv_first_wgrad(const float* in0, int C0, const float* in1, int C1, const float* dz, int lddz, float* dw,
                                       float* workspace, size_t workspace_floats, int B, int H, int W, int Cout, void* stream) {
-    FSDET_CHECK_ARG(in0 && dz && dw && workspace && C0 > 0 && C1 >= 0 && (C1 == 0 || in1) && C0 + C1 <= 4,
+    FSDET_CHECK_ARG(in0 && dz && dw && workspace && C0 > 0 && C1 >= 0 && (C1 == 0 || in1) && C0 + C1 <= 8,
                     "conv_first_wgrad: bad inputs");
     FSDET_CHECK_ARG(Cout > 0 && Cout <= 32 && Cout % 4 == 0 && lddz % 4 == 0, "conv_first_wgrad: Cout=%d lddz=%d", Cout, lddz);
     FSDET_CHECK_ARG(aligned16(dz) && aligned16(dw) && aligned16(workspace), "conv_first_wgrad: alignment");
+    const int nq = first_quads(C0 + C1);
     const int ctas = first_wgrad_ctas(B, H);
-    FSDET_CHECK_ARG(workspace_floats >= (size_t)ctas * FW_SEG * Cout * 36, "conv_first_wgrad: workspace too small");
+    FSDET_CHECK_ARG(workspace_floats >= fsdet_conv_first_wgrad_workspace_floats_cin(B, H, W, C0 + C1, Cout),
+                    "conv_first_wgrad: workspace too small");
     if (ctas == 0) return 0;
-    const size_t smem = ((size_t)FW_SLOTS * (W + 2) * 4 + (size_t)2 * W * 32) * sizeof(float);
-    FSDET_CHECK_ARG(smem <= 227 * 1024, "conv_first_wgrad: image width %d too large", W);
+    FSDET_CHECK_ARG(fsdet_conv_first_wgrad_supported(C0 + C1, W), "conv_first_wgrad: image width %d too large for %d channels", W,
+                    C0 + C1);
     cudaStream_t s = (cudaStream_t)stream;
-    {   // the opt-in ceiling (227 KB), per launch like every other kernel of the library: no cached state, and never lowered under
-        // a graph that was captured at a wider image
-        cudaError_t e = cudaFuncSetAttribute(conv_first_wgrad_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        if (e != cudaSuccess) { set_error("conv_first_wgrad: %s", cudaGetErrorString(e)); return (int)e; }
-    }
-    // scalar FFMA flavour (the packed one is register-bandwidth bound here: 900 us vs 873 us)
-    conv_first_wgrad_kernel<false><<<ctas, FW_THREADS, smem, s>>>(in0, C0, in1, C1, dz, lddz, workspace, B, H, W, Cout);
-    int st = launch_status("conv_first_wgrad");
+    int st = nq == 1 ? launch_first_wgrad<1>(in0, C0, in1, C1, dz, lddz, workspace, B, H, W, Cout, ctas, s)
+                     : launch_first_wgrad<2>(in0, C0, in1, C1, dz, lddz, workspace, B, H, W, Cout, ctas, s);
     if (st) return st;
-    long long n4 = (long long)Cout * 36 / 4;
+    st = launch_status("conv_first_wgrad");
+    if (st) return st;
+    long long n4 = (long long)Cout * 9 * nq;
     first_wgrad_reduce_kernel<<<(unsigned)n4, 128, 0, s>>>(reinterpret_cast<const float4*>(workspace), reinterpret_cast<float4*>(dw),
-                                                           (int)n4, ctas * FW_SEG);
+                                                           (int)n4, ctas * first_wgrad_seg(nq));
     return launch_status("conv_first_wgrad_reduce");
 }

@@ -10,7 +10,8 @@ work of the WHOLE batch is one `fsdet_augment_batch` launch (+ one `fsdet_box_ma
   DetectionBatcher   query images + targets: multi-scale schedule (dataset.py:223-245), data_augmentation,
                      fill_truth_detection(_meta)
   MetaBatcher        support images + masks: get_metain (dataset.py:423-445) incl. its re-draw loop, get_img_mask
-                     (dataset.py:378-398) for metain_type 1/2
+                     (dataset.py:378-398) for metain_type 1/2 and the cropped-object inputs 3/4 (a second augmentation
+                     launch resizes the mask rectangle of each augmented image to full size)
 
 The few-shot list construction (build_dataset / load_metadict / build_fewset, MetaDataset's index) lives in lists.py;
 both classes here take already-built lists.  Entries may be image
@@ -167,15 +168,18 @@ class DetectionBatcher(object):
 
 
 class MetaBatcher(object):
-    """MetaDataset.__getitem__ / get_metain (dataset.py:400-445, 519-530) a batch at a time, metain_type 1 or 2.
+    """MetaDataset.__getitem__ / get_metain (dataset.py:400-445, 519-530) a batch at a time.
 
     metalines[c]: the support pool of class c - image paths, or (uint8 array, boxes [k, 4..5] of that class) pairs;
     inds: sequence of (clsid, metaind) like MetaDataset.inds.  `batch(indices)` returns (metax float32 CUDA
-    [n, 3, S, S], mask float32 CUDA [n, 1, S, S][, clsids])."""
+    [n, C, S, S], mask float32 CUDA [n, 1, S, S][, clsids]).  C = 3 for metain_type 1 / 2 (the image); 6 for 3 / 4
+    (the image, then its mask rectangle cropped and resized to S x S: dataset.py:386-390).  The mask comes back for
+    every type, as in the reference; the network concatenates it for types 2 and 3 only."""
 
     def __init__(self, metalines, inds, classes=None, train=False, ensemble=False, with_ids=False, filter=None):
-        if cfg.metain_type not in (1, 2):
-            raise NotImplementedError('metain_type %r (the cropped-object inputs 3/4 are not used by the shipped cfgs)' % cfg.metain_type)
+        if cfg.metain_type not in (1, 2, 3, 4):
+            raise NotImplementedError('metain_type %r' % cfg.metain_type)
+        self.crop = cfg.metain_type in (3, 4)
         self.metalines, self.inds = metalines, list(inds)
         self.classes = classes if classes is not None else (cfg.base_classes if train else cfg.classes)
         self.train, self.ensemble, self.with_ids, self.filter = train, ensemble, with_ids, filter
@@ -249,8 +253,16 @@ class MetaBatcher(object):
 
     def finish(self, prepared):
         pixels, params, rects, clsids = prepared
-        metax = I.augment_batch(pixels, self.meta_shape, params, filter=self.filter)
         n = len(pixels)
+        if self.crop:
+            W, H = self.meta_shape
+            metax = torch.empty(n, 6, H, W, dtype=torch.float32, device=I._default_device())
+            _, u8 = I.augment_batch(pixels, self.meta_shape, params, filter=self.filter, out=metax[:, :3], return_uint8=True)
+            # img.crop(mask rect).resize(img.size) of the augmented uint8 image, same resampling filter
+            I.augment_batch([u8[i] for i in range(n)], self.meta_shape, [I.crop_params(r) for r in rects.tolist()],
+                            filter=self.filter, out=metax[:, 3:])
+        else:
+            metax = I.augment_batch(pixels, self.meta_shape, params, filter=self.filter)
         w, h = self.mask_shape
         mask = torch.empty(n, 1, h, w, dtype=torch.float32, device=metax.device)
         I.call('fsdet_box_masks', I.ptr(rects.to(metax.device, non_blocking=True)), n, h, w, I.ptr(mask), I._st())

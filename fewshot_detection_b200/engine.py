@@ -358,7 +358,7 @@ class NetRunner(object):
         flops = 2.0 * x.npix * cout * k * k * cin
         if x.nchw is not None:
             in0, c0, in1, c1 = x.nchw
-            assert bias is None and not acc and cin == 4 and k == 3
+            assert bias is None and not acc and cin == _round_up(c0 + c1, 4) and cin <= 8 and k == 3
             if stat_rows_out is not None:   # BatchNorm partial rows straight from the kernel's registers (no pass over z)
                 self._timed('first_fwd', flops, 'fsdet_conv_first_fwd_stats', ptr(in0), c0, ptr(in1), c1, ptr(w_ohwi), z.ptr, z.ld,
                             x.B, x.H, x.W, cout, ptr(stat_rows_out), st)
@@ -527,9 +527,11 @@ class NetRunner(object):
         in0 = inputs[0].contiguous()
         in1 = inputs[1].contiguous() if c1 else None
         if (first is not None and first.kind == 'conv' and not first.dynamic and first.k == 3 and first.cout <= 32
-                and first.cout % 4 == 0 and self.in_ch <= 4):
-            # the first convolution reads the NCHW input directly (no NHWC copy of the images)
-            xin = Act(None, 0, 4, B, H, W, needs_grad=False, dev=dev)
+                and first.cout % 4 == 0 and self.in_ch <= 8 and _lib.lib.fsdet_conv_first_wgrad_supported(self.in_ch, W)):
+            # the first convolution reads the NCHW input directly (no NHWC copy of the images); weights and their
+            # gradient carry in_cpad channels (4 for image + mask, 8 for the cropped-object inputs of metain_type 3 / 4,
+            # whose weight-gradient staging outgrows shared memory past W = 518: those take the NHWC path)
+            xin = Act(None, 0, self.in_cpad, B, H, W, needs_grad=False, dev=dev)
             xin.nchw = (in0, c0, in1, c1)
         else:
             xin = Act.new(B, H, W, self.in_cpad, dev, needs_grad=False)
@@ -982,7 +984,7 @@ class NetRunner(object):
             return
         if x.nchw is not None:
             in0, c0, in1, c1 = x.nchw
-            nws = _lib.lib.fsdet_conv_first_wgrad_workspace_floats(x.B, x.H, x.W, cout)
+            nws = _lib.lib.fsdet_conv_first_wgrad_workspace_floats_cin(x.B, x.H, x.W, c0 + c1, cout)
             ws = _empty(max(nws, 4), device=dev)
             self._timed('first_wgrad', flops, 'fsdet_conv_first_wgrad', ptr(in0), c0, ptr(in1), c1, dz.ptr, dz.ld, ptr(out_tensor),
                         ptr(ws), nws, x.B, x.H, x.W, cout, st)

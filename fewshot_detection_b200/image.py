@@ -166,7 +166,8 @@ def marshal_params(sizes, params, W, H):
 
 def augment_batch(images, shape, params, filter=None, device=None, out=None, return_uint8=False):
     """One launch for a batch: images[i] (uint8 [h, w, 3]) -> out[i] float32 [3, H, W] under params[i] (a dict from
-    draw_augmentation / identity_augmentation).  shape = (W, H) like the reference's `shape` argument."""
+    draw_augmentation / identity_augmentation).  shape = (W, H) like the reference's `shape` argument.
+    `out` may be a channel slice of a larger NCHW tensor (e.g. t[:, 3:6]): each out[i] must be contiguous."""
     if not torch.cuda.is_available():
         raise RuntimeError('augment_batch runs on the GPU only (no CPU fallback)')
     device = _default_device() if device is None else torch.device(device)
@@ -195,10 +196,14 @@ def augment_batch(images, shape, params, filter=None, device=None, out=None, ret
         out = torch.empty(n, 3, H, W, dtype=torch.float32, device=device)
     else:
         assert out.device.type == device.type and out.dtype == torch.float32 and tuple(out.shape) == (n, 3, H, W) \
-            and out.is_contiguous()
+            and out.stride()[1:] == (H * W, W, 1) and (n <= 1 or out.stride(0) >= 3 * H * W)
     u8 = torch.empty(n, H, W, 3, dtype=torch.uint8, device=device) if return_uint8 else None
-    call('fsdet_augment_batch', ptr(ptrs), ptr(geom_d), ptr(color_d), n, W, H, kmax, int(filter), ptr(ws), ws_bytes,
-         ptr(out), ptr(u8), ptr(status), _st())
+    if out.is_contiguous():
+        call('fsdet_augment_batch', ptr(ptrs), ptr(geom_d), ptr(color_d), n, W, H, kmax, int(filter), ptr(ws), ws_bytes,
+             ptr(out), ptr(u8), ptr(status), _st())
+    else:
+        call('fsdet_augment_batch_pitched', ptr(ptrs), ptr(geom_d), ptr(color_d), n, W, H, kmax, int(filter), ptr(ws),
+             ws_bytes, ptr(out), int(out.stride(0)), ptr(u8), ptr(status), _st())
     if return_uint8:
         return out, u8
     return out
@@ -397,6 +402,15 @@ def mask_rect(box, w, h):
     x2 = int(min(w, round((box[0] + box[2] / 2) * w)))
     y2 = int(min(h, round((box[1] + box[3] / 2) * h)))
     return x1, y1, x2, y2
+
+
+def crop_params(rect):
+    """Augmentation parameters of `img.crop(rect).resize(img.size)` (dataset.py:387, the cropped-object input of
+    metain_type 3 / 4) for the augmented uint8 support image: crop at the mask rectangle, no flip, no colour change."""
+    x1, y1, x2, y2 = (int(v) for v in rect)
+    p = identity_augmentation(x2 - x1, y2 - y1)
+    p['pleft'], p['ptop'] = x1, y1
+    return p
 
 
 def box_masks(boxes, w, h, device=None):

@@ -74,19 +74,24 @@ int fsdet_conv_wgrad(const float* x, int ldx, const float* dz, int lddz, float* 
                      size_t workspace_floats, int B, int H, int W, int Cin, int Cout, int ksize, void* stream);
 size_t fsdet_conv_wgrad_workspace_floats(int B, int H, int W, int Cin, int Cout, int ksize);
 /* First layer, read straight from the reference-facing NCHW tensors (in0 [B,C0,H,W] and optionally in1
- * [B,C1,H,W] = the support branch's torch.cat([metax, mask], 1); C0+C1 <= 4; Cout <= 32; 3x3, pad 1):
- * forward z NHWC fp32 with weights zero-padded to [Cout][9][4]; weight gradient dw [Cout][9][4].
- * HBM-bound kernels; workspace float [fsdet_conv_first_wgrad_workspace_floats()]. */
-int fsdet_conv_first_fwd(const float* in0, int C0, const float* in1, int C1, const float* w_pad4, float* z, int ldz,
+ * [B,C1,H,W] = the support branch's torch.cat([metax, mask], 1); C0+C1 <= 8; Cout <= 32; 3x3, pad 1):
+ * forward z NHWC fp32 with weights zero-padded to [Cout][9][P]; weight gradient dw [Cout][9][P], its padding channels
+ * written as zeros.  Channel pitch P = 4 when C0+C1 <= 4 (image + mask), 8 when C0+C1 is 5..8 (image + cropped object
+ * [+ mask], metain_type 3 / 4).  HBM-bound kernels; workspace float [fsdet_conv_first_wgrad_workspace_floats_cin()]
+ * (fsdet_conv_first_wgrad_workspace_floats() = the same for Cin <= 4).  The weight gradient stages x rows and dz rows
+ * in shared memory: fsdet_conv_first_wgrad_supported(Cin, W) says whether they fit (8 channels: W <= 518). */
+int fsdet_conv_first_fwd(const float* in0, int C0, const float* in1, int C1, const float* w_pad, float* z, int ldz,
                          int B, int H, int W, int Cout, void* stream);
 /* The same convolution with the train-mode BatchNorm partial rows taken from the values in registers: stat_partial float
  * [fsdet_conv_first_stat_rows(B, H, W)][4*Cout] = (sum | sum of squares | min | max) per CTA - no fsdet_colstats pass. */
 int fsdet_conv_first_stat_rows(int B, int H, int W);
-int fsdet_conv_first_fwd_stats(const float* in0, int C0, const float* in1, int C1, const float* w_pad4, float* z, int ldz,
+int fsdet_conv_first_fwd_stats(const float* in0, int C0, const float* in1, int C1, const float* w_pad, float* z, int ldz,
                                int B, int H, int W, int Cout, float* stat_partial, void* stream);
 int fsdet_conv_first_wgrad(const float* in0, int C0, const float* in1, int C1, const float* dz, int lddz, float* dw,
                            float* workspace, size_t workspace_floats, int B, int H, int W, int Cout, void* stream);
 size_t fsdet_conv_first_wgrad_workspace_floats(int B, int H, int W, int Cout);
+size_t fsdet_conv_first_wgrad_workspace_floats_cin(int B, int H, int W, int Cin, int Cout);
+int fsdet_conv_first_wgrad_supported(int Cin, int W);
 /* The same first block (conv 3x3 from <= 4 NCHW input channels into Cout <= 32 + train-mode BatchNorm + LeakyReLU +
  * MaxPool 2/2) WITHOUT storing its pre-BN output: every pass recomputes it from the input images with a tcgen05 GEMM
  * per 128-pixel tile (csrc/conv_first_tc.cuh).  Needs H % 8 == 0, W % 16 == 0 (fsdet_conv_first_tc_supported).
@@ -388,6 +393,13 @@ size_t fsdet_augment_workspace_bytes(int n, int W, int H, int kmax);
 int fsdet_augment_batch(const uint8_t* const* src, const int32_t* geom, const double* color, int n, int W, int H,
                         int kmax, int filter, void* workspace, size_t workspace_bytes, float* out, uint8_t* out_u8,
                         int32_t* status, void* stream);
+/* The same with image i written at out + i * out_pitch floats (out_pitch >= 3*H*W), so that several launches can fill
+ * the channel groups of one [n][C][H][W] tensor.  fsdet_augment_batch = out_pitch 3*H*W.  The cropped-object channels
+ * of metain_type 3 / 4 (dataset.py:378-398, `img.crop(rect).resize(img.size)`) are a second launch over the first
+ * launch's out_u8 with geom {W, H, x1, y1, x2 - x1, y2 - y1, 0, 0}, into channels 3..5 of a 6-channel tensor. */
+int fsdet_augment_batch_pitched(const uint8_t* const* src, const int32_t* geom, const double* color, int n, int W, int H,
+                                int kmax, int filter, void* workspace, size_t workspace_bytes, float* out, size_t out_pitch,
+                                uint8_t* out_u8, int32_t* status, void* stream);
 /* dataset.MetaDataset.get_img_mask (dataset.py:378-398): out float32 [n][H][W] = 1 inside rects[i] = {x1, y1, x2, y2}
  * (half-open, already rounded and clamped by the caller as the reference does), else 0. */
 int fsdet_box_masks(const int32_t* rects, int n, int H, int W, float* out, void* stream);

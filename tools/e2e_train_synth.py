@@ -3,7 +3,7 @@
 throw-away VOC-shaped directory: JPEG files + Darknet label files + image list + per-class support dict + .data file +
 .cfg files, base-training protocol of cfg/metayolo.data (15 base classes, novel split 0, neg = 1, multi-scale on).
 
-    python tools/e2e_train_synth.py [n_images] [epochs] [out.json]              (one GPU)
+    python tools/e2e_train_synth.py [n_images] [epochs] [out.json] [--metain-type N]  (one GPU; N = 2 by default)
     torchrun --nproc-per-node 2 tools/e2e_train_synth.py ...                    (one process per GPU)
 
 Prints the driver's log, then one JSON line: images/s of the whole loop (file decode, augmentation, graph-replayed
@@ -67,6 +67,11 @@ def make_dataset(root, n, seed=0):
 
 
 def main():
+    metain_type = 2                 # --metain-type N: the support-input form written to the .data file (1..4)
+    if '--metain-type' in sys.argv:
+        i = sys.argv.index('--metain-type')
+        metain_type = int(sys.argv[i + 1])
+        del sys.argv[i:i + 2]
     n = int(sys.argv[1]) if len(sys.argv) > 1 else 512
     epochs = int(sys.argv[2]) if len(sys.argv) > 2 else 3
     outp = sys.argv[3] if len(sys.argv) > 3 else None
@@ -87,11 +92,11 @@ def main():
         nsamples_all = len(f.readlines())
     det[0]['max_batches'] = str(max(1, (epochs - 1) * nsamples_all // batch))     # max_epochs = max_batches*batch//nsamples + 1
     netcfg.write_cfg(det, os.path.join(root, 'dyn.cfg'))
-    netcfg.write_cfg(netcfg.reweighting_net_blocks(), os.path.join(root, 'rw.cfg'))
+    netcfg.write_cfg(netcfg.reweighting_net_blocks(), os.path.join(root, 'rw.cfg'))   # channels follow metain_type
     backup = os.path.join(root, 'backup')
     with open(os.path.join(root, 'meta.data'), 'w') as f:
-        f.write('metayolo=1\nmetain_type=2\ndata=voc\nneg = 1\nrand = 0\nnovel = %s\nnovelid = 0\nmeta = %s\ntrain = %s\n'
-                'backup = %s\ngpus=%s\n' % (os.path.join(root, 'novels.txt'), os.path.join(root, 'lists', 'dict_full.txt'),
+        f.write('metayolo=1\nmetain_type=%d\ndata=voc\nneg = 1\nrand = 0\nnovel = %s\nnovelid = 0\nmeta = %s\ntrain = %s\n'
+                'backup = %s\ngpus=%s\n' % (metain_type, os.path.join(root, 'novels.txt'), os.path.join(root, 'lists', 'dict_full.txt'),
                                            os.path.join(root, 'lists', 'train.txt'), backup, ','.join(str(i) for i in range(world))))
     import importlib.util
     spec = importlib.util.spec_from_file_location('train_meta_b200', os.path.join(ROOT, 'tools', 'train_meta_b200.py'))
@@ -113,12 +118,12 @@ def main():
     # initial weights: the reference starts from a pretrained trunk; a purely random detector emits box sizes e^N(0, s)
     # that blow the w/h loss up within a few steps.  Write a Darknet weight file (exercises save_weights / load_weights)
     # whose head convolution is scaled down so that training starts from near-zero box offsets.
-    wfile = os.path.join(root, 'init.weights')
+    wfile = os.path.join(root, 'init.weights' if metain_type == 2 else 'init_in%d.weights' % metain_type)
     if rank == 0 and not os.path.exists(wfile):
         import torch
         from fewshot_detection_b200.darknet_meta import Darknet
         torch.manual_seed(0)
-        m0 = Darknet(det, netcfg.reweighting_net_blocks())
+        m0 = Darknet(det, netcfg.reweighting_net_blocks(channels={1: 3, 2: 4, 3: 7, 4: 6}[metain_type]))
         head = [mod for mod in m0.models if isinstance(mod, torch.nn.Sequential)][-1][0]
         with torch.no_grad():
             head.weight.mul_(0.02)
@@ -136,13 +141,15 @@ def main():
     rc = cli.main()
     total = time.time() - t0
     if rank == 0:
+        from fewshot_detection_b200.cfg import _backup_dir
+        bdir = _backup_dir({'backup': backup}, 0)
         steps = sum(nb for nb, _ in marks)
         steady = marks[1:] if len(marks) > 1 else marks
-        line = {'rc': rc, 'world': world, 'images': n, 'global_batch': batch, 'epochs': len(marks), 'steps': steps,
+        line = {'rc': rc, 'world': world, 'images': n, 'metain_type': metain_type, 'backup_dir': bdir, 'global_batch': batch, 'epochs': len(marks), 'steps': steps,
                 'loop_images_per_s': steps * batch / sum(t for _, t in marks),
                 'steady_images_per_s': sum(nb for nb, _ in steady) * batch / sum(t for _, t in steady),
                 'epoch_seconds': [round(t, 3) for _, t in marks], 'wall_s_incl_setup': total,
-                'weights_saved': sorted(os.listdir(backup + '_novel0_neg1')) if os.path.isdir(backup + '_novel0_neg1') else
+                'weights_saved': sorted(os.listdir(bdir)) if os.path.isdir(bdir) else
                 sorted(os.listdir(backup)) if os.path.isdir(backup) else []}
         print(json.dumps(line))
         if outp:

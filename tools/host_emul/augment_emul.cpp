@@ -12,9 +12,9 @@ void set_error(const char*, ...) {}
 
 using namespace fsdet;
 
-extern "C" int emul_augment_batch(const uint8_t* const* src, const int32_t* geom, const double* color, int n, int W, int H,
-                                  int kmax, int filter, int32_t* tables, uint8_t* luts, float* out, uint8_t* out_u8,
-                                  int32_t* status) {
+extern "C" int emul_augment_batch_pitched(const uint8_t* const* src, const int32_t* geom, const double* color, int n, int W,
+                                          int H, int kmax, int filter, int32_t* tables, uint8_t* luts, float* out,
+                                          long long out_pitch, uint8_t* out_u8, int32_t* status) {
     const int L = W > H ? W : H;
     *status = 0;
     const int setup_threads = 2 * L > 768 ? 2 * L : 768;
@@ -22,9 +22,15 @@ extern "C" int emul_augment_batch(const uint8_t* const* src, const int32_t* geom
                         [&]() { augment_setup_kernel(geom, color, n, W, H, L, kmax, filter, tables, luts, status); });
     AugArgs p;
     p.src = src; p.geom = geom; p.tables = tables; p.luts = luts; p.out = out; p.out_u8 = out_u8;
-    p.n = n; p.W = W; p.H = H; p.L = L; p.kmax = kmax; p.filter = filter;
+    p.n = n; p.W = W; p.H = H; p.L = L; p.kmax = kmax; p.filter = filter; p.out_pitch = out_pitch;
     emul::launch_serial(dim3(ceil_div((long long)W * H, kAugThreads), n), dim3(kAugThreads), [&]() { augment_kernel(p); });
     return 0;
+}
+
+extern "C" int emul_augment_batch(const uint8_t* const* src, const int32_t* geom, const double* color, int n, int W, int H,
+                                  int kmax, int filter, int32_t* tables, uint8_t* luts, float* out, uint8_t* out_u8,
+                                  int32_t* status) {
+    return emul_augment_batch_pitched(src, geom, color, n, W, H, kmax, filter, tables, luts, out, 3LL * W * H, out_u8, status);
 }
 
 // all 2^24 (a, b, c) byte triples through the two colour conversions: out[(a*65536 + b*256 + c)*3 ..]
